@@ -2,6 +2,7 @@
 """bench.py -- env-steps/sec of the MetaGym hot path on N B200s of one node (BASELINE.json metric by default).
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--workload quadrotor|maze3d|mixed] [--impl reference]
+                    [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N --master-addr 127.0.0.1 --master-port P \
            bench.py --gpus N --steps K --warmup W [--workload ...]
 
@@ -20,9 +21,17 @@ Workloads (one process per GPU, envs sharded by global index, no data-path colle
             (kernel-side NVLink peer stores; NCCL arena all-gather reported beside it).  One step = one env-step of
             every env (a chunk is 32 steps).
 
-Timing (every workload): the K-step block is captured in CUDA graphs (any K: no eager launches inside the timed
-region) and the block is repeated R times so that the timed region lasts >= 50 ms; `ms_per_step` = timed time /
-(R x K).  CUDA events on the launching stream, barrier + synchronize on both sides, max over ranks.
+Timing (every workload): the timed region is exactly K steps.  quadrotor / maze3d: the K-step block is captured in
+CUDA graphs of at most 256 launches (any K: no eager launches inside the timed region) after one untimed lead-in
+step that keeps the timed steps in steady state, replayed ceil(W / K) times as warm-up and once timed; mixed: max(2, ceil(W / 32)) warm-up chunks, then K / 32 timed chunks (K must be a
+multiple of 32).  `ms_per_step` = timed time / K.  CUDA events on the launching stream, barrier + synchronize on both
+sides, max over ranks.  How many steps run before and inside the timed region depends on the arguments only, so
+with the same arguments every run computes the same outputs.
+
+--dump-outputs DIR: after the timed steps, rank 0 writes what its timed path computed in its last step, the arrays a
+caller of env.step() (mixed: of the fused rollouts, last step of the no-exchange chunk loop) receives, as
+DIR/<name>.npy in float32 (float64 where the engine returns float64).  Above 64 MB in all, a fixed seeded sample of
+envs is written instead, with the sampled env indices in DIR/<name>_env_index.npy.
 
   value     device-resident inputs/outputs.  quadrotor: actions are read from and observations written to rollout buffers
             [32, n, .] (obs 160 MB > 126 MB L2: never L2-hot; the 6 MB recurrent state stays in L2 between steps).
@@ -46,6 +55,9 @@ import time
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
+# the benchmark writes nothing into the tree it runs from (the CPU arm's spawned workers inherit the variable)
+sys.dont_write_bytecode = True
+os.environ["PYTHONDONTWRITEBYTECODE"] = "1"
 
 N_ENVS_PER_GPU = 65536
 DT, NT, N_TASKS = 0.005, 1000, 64
@@ -57,6 +69,8 @@ MIN_TIMED_MS = 50.0
 MAZE3D_BYTES = 128 * 128 * 3 + 1630      # SURVEY.md 8d: uint8 frame + per-env maze state
 MAZE2D_BYTES = 160
 QUAD_HOVER_ROLLOUT_BYTES = 85            # SURVEY.md 8d fused T-step rollout: action 16 + obs 64 + rew 4 + done 1
+MIXED_T = 32                             # steps per fused rollout chunk of the mixed workload
+DUMP_MAX_BYTES = 64 * 10 ** 6
 
 WORKLOADS = {
     "quadrotor": {
@@ -129,6 +143,31 @@ class ClockSampler(object):
                     reasons.add(name)
         return {"sm_mhz": statistics.median(sm) if sm else None, "sm_max_mhz": max(mx) if mx else None,
                 "reasons": sorted(reasons), "samples": len(sm)}
+
+    def close(self):
+        """Make sure no nvidia-smi outlives the benchmark, also when a leg raised before stop()."""
+        if self.proc is not None and self.proc.poll() is None:
+            self.proc.terminate()
+            self.proc.wait()
+
+
+def dump_outputs(path, arrays):
+    """arrays: name -> host array with the env axis first.  Writes <path>/<name>.npy in float32 (float64 stays
+    float64).  Above DUMP_MAX_BYTES in all, the same fraction of envs of every array is kept, drawn with a fixed seed,
+    and the kept env indices go to <name>_env_index.npy."""
+    import numpy as np
+    os.makedirs(path, exist_ok=True)
+    out = {k: v.astype(np.float64 if v.dtype == np.float64 else np.float32) for k, v in arrays.items()}
+    total = sum(v.nbytes for v in out.values())
+    if total > DUMP_MAX_BYTES:
+        frac = DUMP_MAX_BYTES / (total + 8.0 * sum(len(v) for v in out.values()))
+        for k in list(out):
+            n = len(out[k])
+            idx = np.sort(np.random.RandomState(0).choice(n, max(1, int(n * frac)), replace=False))
+            out[k] = np.ascontiguousarray(out[k][idx])
+            out[k + "_env_index"] = idx.astype(np.float64)
+    for k, v in out.items():
+        np.save(os.path.join(path, k + ".npy"), v)
 
 
 # ---------------------------------------------------------------------------------------------------------------
@@ -239,54 +278,66 @@ def run_reference(args, rank, world):
 # graph-replayed K-step blocks
 # ---------------------------------------------------------------------------------------------------------------
 class GraphedBlock(object):
-    """K steps of `enqueue(t)` captured in CUDA graphs so that ANY K is replayed from graphs (no eager launch in a timed
-    region).  K <= 256: one graph holds m = 256 // K whole blocks (so that consecutive blocks keep their programmatic
-    dependent-launch edges); K > 256: graphs of 256 steps + one remainder graph."""
+    """Exactly K steps of `enqueue(t)` captured in CUDA graphs so that ANY K is replayed from graphs (no eager launch in
+    a timed region).  The K steps are cut into pieces of 256 (t = 0..255) and a remainder (t = 0..K % 256 - 1); the
+    first piece is a graph that begins with one untimed lead-in step, the last one a graph that ends by recording `end`,
+    and the pieces between are replays of one 256-step graph.  `start` is recorded on a branch that waits for the
+    lead-in step alone, so the kernels keep their programmatic dependent-launch chain and `elapsed_ms()` of a replay is
+    the K steps in steady state: no graph launch, no first-kernel launch latency.  A replay runs `steps` = K + 1 steps;
+    `last_t` is the t of the block's last step."""
     UNIT = 256
 
     def __init__(self, torch, dev, enqueue, K, warm_steps):
         self.torch, self.K = torch, K
+        self.start = torch.cuda.Event(enable_timing=True, external=True)     # recorded by a node of the graph
+        self.end = torch.cuda.Event(enable_timing=True, external=True)
         self.stream = torch.cuda.Stream(device=dev)
-        self.graphs = []           # (graph, steps)
+        self.branch = torch.cuda.Stream(device=dev)
+        self.steps = K + 1
         self.stream.wait_stream(torch.cuda.current_stream(dev))     # side stream: ordered after the caller's pending work
         with torch.cuda.stream(self.stream):
             for t in range(max(3, warm_steps)):
                 enqueue(t)
             self.stream.synchronize()
-            if K <= self.UNIT:
-                self.blocks_per_replay = max(1, self.UNIT // K)
-                self.plan = [(self._capture(enqueue, K * self.blocks_per_replay), 1)]
-            else:
-                self.blocks_per_replay = 1
-                self.plan = [(self._capture(enqueue, self.UNIT), K // self.UNIT)]
-                if K % self.UNIT:
-                    self.plan.append((self._capture(enqueue, K % self.UNIT), 1))
+            sizes = [self.UNIT] * (K // self.UNIT) + ([K % self.UNIT] if K % self.UNIT else [])
+            self.plan = [(self._capture(enqueue, sizes[0], start=True, end=len(sizes) == 1), sizes[0], 1)]
+            if len(sizes) > 2:                                       # (graph, steps, replays)
+                self.plan.append((self._capture(enqueue, self.UNIT), self.UNIT, len(sizes) - 2))
+            if len(sizes) > 1:
+                self.plan.append((self._capture(enqueue, sizes[-1], end=True), sizes[-1], 1))
+        self.last_t = sizes[-1] - 1
         torch.cuda.synchronize(dev)
 
-    def _capture(self, enqueue, steps):
+    def _capture(self, enqueue, steps, start=False, end=False):
         g = self.torch.cuda.CUDAGraph()
         with self.torch.cuda.graph(g, stream=self.stream):
+            if start:
+                enqueue(0)                                  # lead-in step
+                self.branch.wait_stream(self.stream)
+                self.start.record(self.branch)
             for t in range(steps):
                 enqueue(t)
+            if start:
+                self.stream.wait_stream(self.branch)        # join the branch before the capture ends
+            if end:
+                self.end.record()
         return g
 
-    def steps_per_replay(self):
-        return self.K * self.blocks_per_replay
+    def elapsed_ms(self):
+        """Device time of the last completed replay of the block."""
+        return self.start.elapsed_time(self.end)
 
     def replay(self, times=1):
-        """`times` x (blocks_per_replay blocks of K steps), on the current stream."""
+        """`times` x K steps, on the current stream."""
         for _ in range(times):
-            for g, reps in self.plan:
+            for g, _, reps in self.plan:
                 for _ in range(reps):
                     g.replay()
 
     def describe(self, what):
-        if self.K <= self.UNIT:
-            return "CUDA graph of %d %s launches (%d blocks of K=%d steps) replayed R times" % (
-                self.steps_per_replay(), what, self.blocks_per_replay, self.K)
-        return "CUDA graphs of %d %s launches x %d%s per K=%d block, block replayed R times" % (
-            self.UNIT, what, self.K // self.UNIT, (" + one of %d" % (self.K % self.UNIT)) if self.K % self.UNIT else "",
-            self.K)
+        sizes = " + ".join("%d x %d" % (reps, steps) for _, steps, reps in self.plan)
+        return "K=%d %s launches after one lead-in in CUDA graphs (replays x launches: %s), replayed once timed" % (
+            self.K, what, sizes)
 
 
 class Ctx(object):
@@ -304,6 +355,7 @@ class Ctx(object):
         if self.world > 1:
             dist.init_process_group("nccl", device_id=self.dev)
         self.peak, self.peak_src = measured_peak_gbs()
+        self.outputs = None
         self.e0 = torch.cuda.Event(enable_timing=True)
         self.e1 = torch.cuda.Event(enable_timing=True)
 
@@ -329,21 +381,23 @@ class Ctx(object):
         return self.max_over_ranks(self.e0.elapsed_time(self.e1))
 
     def time_block(self, block, W):
-        """Warm up, size R for a >= 50 ms timed region (same R on every rank), time it.  -> dict"""
+        """ceil(W / K) warm-up replays of the block (every graph of it has run before the timed one), then one timed
+        replay: exactly K steps, timed by the events the block's graphs record.  -> dict"""
         K = block.K
-        block.replay(max(1, -(-W // block.steps_per_replay())))
-        probe = self.timed(lambda: block.replay(1))
-        R = max(1, int(math.ceil(1.05 * MIN_TIMED_MS / max(probe, 1e-3))))
-        for _ in range(4):
-            t_wall0 = time.time()
-            ms = self.timed(lambda: block.replay(R))      # max over ranks: every rank sees the same ms and takes the same branch
-            t_wall1 = time.time()
-            if ms >= MIN_TIMED_MS:
-                break
-            R = int(math.ceil(R * 1.25 * MIN_TIMED_MS / max(ms, 1e-3)))   # a lone replay over-estimates: re-time with more
-        steps = R * block.steps_per_replay()
-        return {"ms": ms, "timed_steps": steps, "repeats": R * block.blocks_per_replay, "ms_per_step": ms / steps,
+        warm = max(1, -(-W // K))
+        self.barrier()
+        t_wall0 = time.time()
+        block.replay(warm + 1)
+        self.barrier()
+        t_wall1 = time.time()
+        ms = self.max_over_ranks(block.elapsed_ms())
+        return {"ms": ms, "timed_steps": K, "repeats": 1, "ms_per_step": ms / K, "warmup_steps": warm * block.steps + 1,
                 "t_wall0": t_wall0, "t_wall1": t_wall1, "K": K}
+
+    def snapshot(self, arrays):
+        """Host copies of the timed path's last-step outputs, kept for --dump-outputs (rank 0)."""
+        if self.args.dump_outputs and self.rank == 0:
+            self.outputs = {k: v.detach().cpu().numpy() for k, v in arrays.items()}
 
     def close(self):
         if self.world > 1:
@@ -385,6 +439,8 @@ def run_quadrotor(ctx, sampler):
 
     block = GraphedBlock(torch, dev, enqueue, K, min(W, G))
     tm = ctx.time_block(block, W)
+    s = block.last_t % G
+    ctx.snapshot({"obs": obs[s], "reward": rew[s], "done": done[s]})
     us_per_launch = tm["ms_per_step"] * 1e3
     value = n * world / (tm["ms_per_step"] * 1e-3)
     achieved = n * BYTES_PER_STEP / (us_per_launch * 1e-6) / 1e9
@@ -482,8 +538,8 @@ def run_quadrotor(ctx, sampler):
     info = {}
     info.update({
         "launch": block.describe("mgb_quad_step") + " (programmatic dependent launch between consecutive steps)",
-        "timed_region": "R x K = %d steps in %.1f ms (>= %.0f ms), CUDA events, max over ranks" % (
-            tm["timed_steps"], tm["ms"], MIN_TIMED_MS),
+        "timed_region": "K = %d steps in %.2f ms after %d warm-up steps, CUDA events, max over ranks" % (
+            tm["timed_steps"], tm["ms"], tm["warmup_steps"]),
         "l2": "rollout buffers obs [32,n,19] f32 = 160 MB > 126 MB L2 (inputs/outputs never L2-hot); "
               "the 6 MB recurrent state is L2-resident by nature of the workload; see extras.streaming "
               "for the 4M-env run whose state streams from HBM",
@@ -598,7 +654,7 @@ def maze_step_rates(ctx):
         env.reset()
         acts = torch.randint(0, 4, (16, n), device=dev, dtype=torch.int32)
         block = GraphedBlock(torch, dev, lambda t: env.step(acts[t % 16]), 64, 8)
-        tm = ctx.time_block(block, 8) if ctx.world == 1 else _time_block_local(ctx, block)
+        tm = _time_block_local(ctx, block)
         us = tm["ms_per_step"] * 1e3
         out[name] = {"value": n / us * 1e6, "unit": "env-steps/s", "us_per_step": us, "timed_steps": tm["timed_steps"],
                      "algorithmic_bytes_per_env_step": nbytes, "frac_of_measured_hbm": n * nbytes / us * 1e-3 / ctx.peak,
@@ -619,9 +675,9 @@ def _time_block_local(ctx, block):
     ctx.e0.record(); block.replay(R); ctx.e1.record()
     torch.cuda.synchronize(ctx.dev)
     ms = ctx.e0.elapsed_time(ctx.e1)
-    steps = R * block.steps_per_replay()
-    return {"ms": ms, "timed_steps": steps, "repeats": R * block.blocks_per_replay, "ms_per_step": ms / steps,
-            "t_wall0": 0, "t_wall1": 0, "K": block.K}
+    steps = R * block.steps
+    return {"ms": ms, "timed_steps": steps, "repeats": R, "ms_per_step": ms / steps, "t_wall0": 0, "t_wall1": 0,
+            "K": block.K}
 
 
 def run_maze3d(ctx, sampler):
@@ -642,8 +698,15 @@ def run_maze3d(ctx, sampler):
     env.step(acts[0])
     torch.cuda.synchronize(dev)
     set_task_s = time.perf_counter() - t0
-    block = GraphedBlock(torch, dev, lambda t: env.step(acts[t % SLOTS]), K, min(W, SLOTS))
+    last = {}
+
+    def enqueue(t):
+        last["out"] = env.step(acts[t % SLOTS])     # the env's own output buffers, the same ones every step
+
+    block = GraphedBlock(torch, dev, enqueue, K, min(W, SLOTS))
     tm = ctx.time_block(block, W)
+    ctx.snapshot(dict(zip(("obs", "reward", "done"), last["out"][:3])))
+    launch = block.describe("mgb_maze_step")
     us = tm["ms_per_step"] * 1e3
     value = n * world / (tm["ms_per_step"] * 1e-3)
     achieved = n * MAZE3D_BYTES / (us * 1e-6) / 1e9
@@ -773,7 +836,9 @@ def run_maze3d(ctx, sampler):
         return None
     cfg = base_config("maze3d", world)
     info = {}
-    info.update({"launch": block_desc_maze(K), "timed_region": "%d steps in %.1f ms" % (tm["timed_steps"], tm["ms"]),
+    info.update({"launch": launch,
+                "timed_region": "K = %d steps in %.2f ms after %d warm-up steps" % (tm["timed_steps"], tm["ms"],
+                                                                                   tm["warmup_steps"]),
                 "renderer": "pose cache (64 tasks): cached static layers + per-step integer compose; see many_tasks for "
                             "the direct raycaster", "set_task_plus_first_step_s": set_task_s,
                 "l2": "frames 50 MB/step written to one buffer (L2 126 MB): outputs may stay L2-resident; the cache of "
@@ -801,10 +866,6 @@ def run_maze3d(ctx, sampler):
     return line
 
 
-def block_desc_maze(K):
-    return "mgb_maze_step launches captured in CUDA graphs (K=%d block, <=256 launches per graph), replayed R times" % K
-
-
 # ---------------------------------------------------------------------------------------------------------------
 # workload: mixed (BASELINE configs[4])
 # ---------------------------------------------------------------------------------------------------------------
@@ -813,9 +874,8 @@ def run_mixed(ctx, sampler):
     from metagym_b200 import BatchedMetaMaze2D, BatchedQuadrotor
     from metagym_b200.rollout import PeerArena, RolloutArena
     NQ = NM = (args.envs or 32768) // 2
-    T = 32
+    T = MIXED_T
     K, W = args.steps, args.warmup
-    chunks = max(1, -(-K // T))
     quad = BatchedQuadrotor(task="hovering_control", dt=0.01, nt=1000, num_envs=NQ, device=ctx.local_rank,
                             squeeze=False, auto_reset=True, env_index_base=rank * NQ)
     maze = BatchedMetaMaze2D(max_steps=200, task_type="ESCAPE", view_grid=1, num_envs=NM, device=ctx.local_rank,
@@ -840,9 +900,9 @@ def run_mixed(ctx, sampler):
     payload = plain.payload_bytes()
     for _ in range(max(2, -(-W // T))):
         collect(plain.views)
-    probe = ctx.timed(lambda: collect(plain.views))
-    reps = max(chunks, int(math.ceil(1.3 * MIN_TIMED_MS / max(probe, 1e-3))))      # a lone probe over-estimates a chunk
+    reps = K // T
     ms_none = ctx.timed(lambda: [collect(plain.views) for _ in range(reps)])
+    ctx.snapshot({k: v[T - 1] for k, v in plain.views.items()})
     results = {"no_exchange": {"value": (NQ + NM) * world * T * reps / (ms_none * 1e-3), "ms_per_chunk": ms_none / reps}}
     how = "none (1 GPU: the chunk is already where the learner is)"
     ms_best, t_wall0 = ms_none, time.time()
@@ -979,6 +1039,8 @@ def main():
     ap.add_argument("--envs", type=int, default=0, help="envs per GPU (default: the workload's BASELINE shape)")
     ap.add_argument("--no-extras", action="store_true", help="skip streaming / fused / e2e / cpu legs")
     ap.add_argument("--cpu-seconds", type=float, default=0.0, help="length of the CPU arm (default 10 s; reference arm 30 s)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the last timed step's outputs to DIR/<name>.npy (float32 / float64, <= 64 MB in all)")
     args = ap.parse_args()
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
@@ -986,13 +1048,20 @@ def main():
     assert args.steps >= 1
     if args.impl == "reference":
         return run_reference(args, rank, world)
+    if args.workload == "mixed" and args.steps % MIXED_T:
+        ap.error("--workload mixed times whole rollout chunks: --steps must be a multiple of %d" % MIXED_T)
 
     ctx = Ctx(args)
     sampler = ClockSampler(ctx.local_rank)
     if ctx.rank == 0:
         sampler.start()
-    line = {"quadrotor": run_quadrotor, "maze3d": run_maze3d, "mixed": run_mixed}[args.workload](ctx, sampler)
+    try:
+        line = {"quadrotor": run_quadrotor, "maze3d": run_maze3d, "mixed": run_mixed}[args.workload](ctx, sampler)
+    finally:
+        sampler.close()
     if ctx.rank == 0:
+        if args.dump_outputs:
+            dump_outputs(args.dump_outputs, ctx.outputs)
         if not args.no_extras:
             line["cpu_baseline"] = cpu_arm(args.workload, float(args.cpu_seconds) if args.cpu_seconds else 10.0)
         print(json.dumps(line), flush=True)

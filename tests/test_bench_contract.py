@@ -42,3 +42,25 @@ def test_reference_arm_other_workload_has_its_own_metric():
     assert d["metric"] == bench.WORKLOADS["maze3d"]["metric"]
     assert d["config"] == bench.base_config("maze3d", 1)
     assert d["cpu_baseline"]["value"] == d["value"] > 0
+
+
+def test_dump_outputs_keeps_a_fixed_sample_under_the_budget(tmp_path):
+    """--dump-outputs: float32 (float64 kept), and above 64 MB the same seeded env sample on every run."""
+    import numpy as np
+    import bench
+    obs = np.random.RandomState(1).randint(0, 256, (1024, 128, 128, 3)).astype(np.uint8)
+    arrays = {"obs": obs, "reward": np.arange(1024, dtype=np.float64), "done": np.arange(1024) % 3 == 0}
+    for d in ("a", "b"):
+        bench.dump_outputs(str(tmp_path / d), arrays)
+    names = sorted(p.name for p in (tmp_path / "a").iterdir())
+    assert names == sorted(k + s for k in arrays for s in (".npy", "_env_index.npy"))
+    assert sum(p.stat().st_size for p in (tmp_path / "a").iterdir()) <= 64 * 10 ** 6
+    for n in names:
+        assert np.array_equal(np.load(tmp_path / "a" / n), np.load(tmp_path / "b" / n))
+    idx = np.load(tmp_path / "a" / "obs_env_index.npy").astype(np.int64)
+    assert np.array_equal(np.load(tmp_path / "a" / "obs.npy"), obs[idx].astype(np.float32))
+    assert np.load(tmp_path / "a" / "reward.npy").dtype == np.float64
+    assert np.load(tmp_path / "a" / "done.npy").dtype == np.float32
+    small = {"obs": np.ones((64, 19), np.float32), "done": np.zeros(64, np.uint8)}
+    bench.dump_outputs(str(tmp_path / "c"), small)
+    assert sorted(p.name for p in (tmp_path / "c").iterdir()) == ["done.npy", "obs.npy"]

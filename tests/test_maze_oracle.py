@@ -101,33 +101,29 @@ def test_continuous_maze_oracle_matches_reference(cont_golden, geom_golden, name
     assert c["done"].sum() >= 1 and (c["rew"] > 0).sum() >= 1
 
 
-@pytest.mark.reference
 def test_oracle_vs_reference_real_textures():
-    """Build container only: the reference renderer with its own PNG textures vs the oracle, random poses."""
+    """The reference renderer with its own PNG textures vs the oracle, random walk at 128x128: every frame bit for bit
+    (SHA-256 of the int32 pixels, whole frames kept for every tenth step), rewards and dones
+    (tests/golden/gen_maze_real_textures.py)."""
+    import hashlib
     import os
-    import sys
-    sys.path.insert(0, os.path.join(os.path.dirname(__file__), "golden"))
-    import _refload
-    if not _refload.reference_available():
-        pytest.skip("reference tree not mounted")
-    import random
-    ns = _refload.load_reference()
-    from metagym_b200.textures import load_texture_dir
-    tex = load_texture_dir(os.path.join(_refload.REF_ROOT, "metagym", "metamaze", "envs", "img"))
-    ns.MAZE_TASK_MANAGER.grounds = tex[0].astype(np.float32)
-    ns.MAZE_TASK_MANAGER.ceil = tex[1]
-    random.seed(5)
-    np.random.seed(5)
-    task = ns.MazeTaskSampler(n=15, allow_loops=True, crowd_ratio=0.35, food_density=0.05)
-    ref = ns.MetaMazeDiscrete3D(enable_render=False, resolution=(128, 128), max_steps=500, task_type="SURVIVAL")
-    ref.set_task(task)
-    ora = OracleMaze("3D", "SURVIVAL", 500, 1, (128, 128), textures=tex)
+    from util import task_from_arrays
+    g = np.load(os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden", "maze_real_textures_golden.npz"))
+    task = task_from_arrays(g["task.walls"], g["task.texts"], g["task.food"], g["task.interval"], g["task.scalars"])
+    ora = OracleMaze("3D", "SURVIVAL", 500, 1, (128, 128), textures=(g["tex.grounds"], g["tex.ceil"]))
     ora.set_task(task)
-    assert np.array_equal(ref.reset(), ora.reset())
-    rng = np.random.RandomState(0)
-    for t in range(60):
-        a = int(rng.randint(4))
-        o1, r1, d1, _ = ref.step(a)
-        o2, r2, d2, _ = ora.step(a)
-        assert np.array_equal(o1, o2), (t, int((o1 != o2).sum()))
-        assert r1 == r2 and d1 == d2
+    kept = {int(t): k for k, t in enumerate(g["kept_idx"])}
+
+    def check(t, obs):
+        if t in kept:
+            ref = g["kept_frames"][kept[t]].astype(np.int32)
+            assert np.array_equal(obs, ref), (t, int((obs != ref).sum()))
+        digest = hashlib.sha256(np.ascontiguousarray(obs, dtype=np.int32).tobytes()).digest()
+        assert digest == g["frame_sha256"][t].tobytes(), t
+
+    check(0, ora.reset())
+    for t, a in enumerate(g["act"]):
+        o2, r2, d2, _ = ora.step(int(a))
+        check(t + 1, o2)
+        assert r2 == g["rew"][t] and d2 == bool(g["done"][t]), t
+    assert len(g["act"]) == 60 and (g["rew"] > 0).sum() >= 1
